@@ -4,6 +4,7 @@ SDXL tile-upscale at 1/2/4/8 B200; blend HBM GB/s").
 
   python bench.py --gpus N --steps K --warmup W              our arm (CUDA kernels)
   python bench.py --impl reference --gpus N --steps K ...    the reference's CPU path (port)
+  python bench.py ... --dump-outputs DIR                      also write what the last timed step computed
 
 A step is one full pass of the hot path over one synthetic canvas: quantise -> per wave
 (crop+LANCZOS kernel, sampler call, LANCZOS-back+composite kernel) -> dequantise.
@@ -16,6 +17,11 @@ number isolates tile ops + transport, which is the path this repo replaces.
 `e2e`     : same metric through the node API (UltimateSDUpscaleDistributed.run) with a
             pinned HOST tensor in and a HOST tensor out -- H2D/D2H inside the timed region.
 `roofline`: dominant kernel (seam blend), algorithmic bytes / CUDA-event time per launch.
+
+--dump-outputs DIR writes rank 0's result of the last timed step as DIR/result.npy (fp32 [B,H,W,3]) when it
+is at most DUMP_MAX_BYTES, else as a fixed sample: DIR/result_sample.npy (fp32) holds the values at the flat
+indices in DIR/result_sample_index.npy (float64), drawn from a generator seeded with 0.  The inputs are seeded,
+so two builds run with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -38,6 +44,23 @@ WORKLOADS = {
     "cfg5_video_17f_4k": (17, 2160, 3840, 512, 32, 8),
 }
 SEED, DENOISE = 123, 0.5
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SAMPLES = 4 << 20          # sampled values (fp32) + their indices (float64): 48 MiB
+
+
+def dump_result(out, path: str) -> None:
+    """Write one result tensor under `path` (see --dump-outputs in the module docstring)."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    flat = out.detach().reshape(-1)
+    if flat.numel() * 4 <= DUMP_MAX_BYTES:
+        np.save(os.path.join(path, "result.npy"), out.detach().to(torch.float32).cpu().numpy())
+        return
+    idx = torch.randint(flat.numel(), (DUMP_SAMPLES,), generator=torch.Generator().manual_seed(0)).sort().values
+    vals = flat[idx.to(flat.device)].to(torch.float32).cpu().numpy()
+    np.save(os.path.join(path, "result_sample.npy"), vals)
+    np.save(os.path.join(path, "result_sample_index.npy"), idx.numpy().astype(np.float64))
 
 
 def make_canvas_cpu(B, H, W):
@@ -344,7 +367,13 @@ def main():
     ap.add_argument("--semantics", default="static", choices=["static", "exact"],
                     help="N > 1: the reference's static mode (default, the headline) or the cooperative single-GPU DAG "
                          "(dist.upscale_exact: bit-identical to N = 1 at any world size; device-resident line only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step under DIR as .npy (a seeded sample when it is large)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs needs the CUDA arm: --impl reference times a bounded sample of the job")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -480,7 +509,14 @@ def main():
     stats = {}
     nvl = NvlinkCounters(local) if world > 1 else None
     nvl0 = nvl.read() if nvl else None
-    ms_step = timed(lambda: step_device(stats), args.steps)
+    last = []
+
+    def timed_step():
+        out = step_device(stats)
+        if args.dump_outputs:
+            last[:] = [out]
+
+    ms_step = timed(timed_step, args.steps)
     nvl1 = nvl.read() if nvl else None
     nvlink = None
     if nvl0 is not None and nvl1 is not None:
@@ -658,6 +694,9 @@ def main():
         if world > 1:
             td.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_result(last[0], args.dump_outputs)
+    del last
 
     peak, peak_src = measured_peak_gbs()
     dom = "blend"

@@ -6,7 +6,7 @@ Outputs (committed, small):
                                   extract_batch_tile_with_padding + calculate_tiles
   tests/golden/single_*.npz       u8 outputs of the reference's process_single_gpu with
                                   the T0 denoiser (inputs are regenerated from seeds)
-  tests/golden/prims.npz          create_tile_mask windows and blend_tile outputs
+  tests/golden/prims.npz          create_tile_mask windows and the window blend_tile wrote (inputs from a seed)
   tests/golden/mask_crop.npz      crop_mask outputs (conditioning masks cut to a tile), u8
   tests/golden/static_ref_index.json   the reference's multi-worker static mode run over HTTP here: the tile
                                   assignment each run ended up with + SHA-256 of the master's u8 result
@@ -186,12 +186,14 @@ def main():
         x1, y1, x2, y2, pw, ph = orc.crop_geometry(W, H, x, y, tw, th, pad, True)
         base = rng.integers(0, 256, (H, W, 3), dtype=np.uint8)
         tile = rng.integers(0, 256, (ph, pw, 3), dtype=np.uint8)
-        out = node.blend_tile(Image.fromarray(base), Image.fromarray(tile), x1, y1, (x2 - x1, y2 - y1), mask, pad)
+        out = np.array(node.blend_tile(Image.fromarray(base), Image.fromarray(tile), x1, y1, (x2 - x1, y2 - y1), mask, pad))
+        outside = out.copy()
+        outside[y1:y2, x1:x2] = base[y1:y2, x1:x2]
+        assert np.array_equal(outside, base), "blend_tile changed pixels outside the crop window"
+        # base and tile are regenerated from the seed by the test; only the window blend_tile wrote is stored
         prims[f"case{i}_params"] = np.array([W, H, x, y, tw, th, blur, pad, x1, y1, x2, y2, pw, ph])
         prims[f"case{i}_mask"] = np.array(mask)
-        prims[f"case{i}_base"] = base
-        prims[f"case{i}_tile"] = tile
-        prims[f"case{i}_out"] = np.array(out)
+        prims[f"case{i}_out_window"] = np.ascontiguousarray(out[y1:y2, x1:x2])
         print("prim", i, (W, H, x, y, blur, pad))
     np.savez_compressed(os.path.join(OUT, "prims.npz"), **prims)
 

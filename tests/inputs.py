@@ -1,6 +1,38 @@
 """Synthetic canvases shared by the golden generator and the tests (values k/255 fp32)."""
+import hashlib
+
 import numpy as np
 import torch
+
+
+def fingerprint(obj):
+    """JSON-comparable form of a nested result: every tensor / array becomes "shape/dtype/sha256", containers are
+    walked (a tuple stays distinct from a list), scalars and strings stay.  What the reference computed is stored in
+    this form under tests/golden/reference_fingerprints.json (oracle/gen_reference_fingerprints.py)."""
+    if isinstance(obj, torch.Tensor):
+        obj = obj.detach().cpu().contiguous().numpy()
+    if isinstance(obj, np.ndarray):
+        a = np.ascontiguousarray(obj)
+        return f"{list(a.shape)}/{a.dtype}/{hashlib.sha256(a.tobytes()).hexdigest()[:32]}"
+    if isinstance(obj, dict):
+        return {str(k): fingerprint(v) for k, v in sorted(obj.items(), key=lambda kv: str(kv[0]))}
+    if isinstance(obj, tuple):
+        return {"tuple": [fingerprint(x) for x in obj]}
+    if isinstance(obj, list):
+        return [fingerprint(x) for x in obj]
+    return obj
+
+
+def reference_fingerprints(test: str) -> dict:
+    """What the reference computed for one side-by-side test, keyed by case (tests/golden/reference_fingerprints.json;
+    empty while the generator is writing it, so that a test then fails on the missing case)."""
+    import json
+    import os
+    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_fingerprints.json")
+    if not os.path.isfile(path):
+        return {}
+    with open(path) as f:
+        return json.load(f)["tests"].get(test, {})
 
 
 def make_input(kind: str, seed: int, B: int, H: int, W: int) -> np.ndarray:

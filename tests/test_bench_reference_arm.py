@@ -41,3 +41,27 @@ def test_reference_arm_http_workers():
     d = json.loads(lines[-1])
     assert d["impl"] == "reference" and d["n_gpus"] == 2 and d["value"] > 0
     assert "aiohttp" in json.dumps(d["cpu_baseline"]) or "HTTP" in json.dumps(d["cpu_baseline"])
+
+
+def test_dump_outputs_is_bounded_and_repeatable(tmp_path):
+    """bench.py --dump-outputs: a small result is written whole; a large one as a fixed seeded sample under 64 MiB."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    small = torch.rand(1, 64, 48, 3)
+    bench.dump_result(small, str(tmp_path / "small"))
+    got = np.load(tmp_path / "small" / "result.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, small.numpy())
+    big = torch.rand(1, 2400, 2400, 3)                       # 69 MB of fp32
+    for d in ("a", "b"):
+        bench.dump_result(big, str(tmp_path / d))
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["result_sample.npy", "result_sample_index.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 << 20
+    idx = np.load(tmp_path / "a" / "result_sample_index.npy")
+    vals = np.load(tmp_path / "a" / "result_sample.npy")
+    assert idx.dtype == np.float64 and vals.dtype == np.float32
+    assert np.array_equal(vals, big.reshape(-1).numpy()[idx.astype(np.int64)])
+    for f in files:
+        assert np.array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f))

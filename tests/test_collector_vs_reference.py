@@ -1,6 +1,7 @@
-"""oracle.collector_combine == the reference's own DistributedCollector arithmetic (worker PNG round trip,
-master decode, _reorder_and_combine_tensors), loaded from /root/reference by oracle/ref_collector.py.
-Skipped where the reference tree is absent; tests/golden/collector_ref.json pins the same there."""
+"""oracle.collector_combine and our audio combination == the reference's own DistributedCollector (worker PNG
+round trip, master decode, _reorder_and_combine_tensors, _combine_audio).  What the reference computed is stored
+in tests/golden/collector_ref.json and tests/golden/reference_fingerprints.json (oracle/ref_collector.py loads the
+reference to regenerate them)."""
 import hashlib
 import json
 import os
@@ -11,6 +12,7 @@ import torch
 
 import ref_collector
 import usdu_oracle as orc
+from inputs import fingerprint, reference_fingerprints
 
 G = os.path.join(os.path.dirname(__file__), "golden")
 CASES = json.load(open(os.path.join(G, "collector_ref.json")))["cases"]
@@ -32,40 +34,44 @@ def test_oracle_collector_matches_golden(case):
     assert list(out.shape) == case["shape"]
 
 
-@pytest.mark.skipif(not ref_collector.available(), reason="reference tree not present")
-@pytest.mark.parametrize("case", CASES, ids=lambda c: c["name"])
-def test_reference_collector_matches_golden_and_oracle(case):
-    master, workers = _inputs(case)
-    ref = ref_collector.combine(master, workers, case["order"], case["delegate"]).numpy()
-    assert hashlib.sha256(np.ascontiguousarray(ref, dtype=np.float32).tobytes()).hexdigest() == case["sha256"]
-    out = orc.collector_combine(master.numpy(), {w: t.numpy() for w, t in workers.items()}, case["order"], case["delegate"])
-    assert np.array_equal(out, ref)
-
-
-@pytest.mark.skipif(not ref_collector.available(), reason="reference tree not present")
-def test_audio_combination_matches_reference():
-    """nodes/collector.py:121-174 side by side with our combine_audio on random piece sets (missing audio,
-    empty waveforms, non-default sample rates, unexpected worker ids)."""
-    from __graft_entry__ import load_package
-    load_package()
-    from comfyui_distributed_b200.nodes.collector import combine_audio
-    collector, _, _ = ref_collector.load()
-    node = collector.DistributedCollectorNode()
-    empty = {"waveform": torch.zeros(1, 2, 1), "sample_rate": 44100}
+def _audio_cases():
+    """200 random piece sets: missing audio, empty waveforms, non-default sample rates, unexpected worker ids."""
     rng = np.random.default_rng(0)
+
+    def piece():
+        k = rng.integers(0, 4)
+        if k == 0:
+            return None
+        n = 0 if k == 1 else int(rng.integers(1, 50))
+        return {"waveform": torch.from_numpy(rng.random((1, 2, n), dtype=np.float32)), "sample_rate": int(rng.choice([44100, 48000, 22050]))}
+
     for _ in range(200):
-        def piece():
-            k = rng.integers(0, 4)
-            if k == 0:
-                return None
-            n = 0 if k == 1 else int(rng.integers(1, 50))
-            return {"waveform": torch.from_numpy(rng.random((1, 2, n), dtype=np.float32)), "sample_rate": int(rng.choice([44100, 48000, 22050]))}
         master = piece()
         ids = ["w1", "w2", "w3", "zz"]
         workers = {w: piece() for w in ids if rng.random() < 0.8}
         order = [w for w in ["w2", "w1", "w3"] if rng.random() < 0.8]
-        ref = node._combine_audio(master, workers, empty, order)
+        yield master, workers, order
+
+
+EMPTY_AUDIO = {"waveform": torch.zeros(1, 2, 1), "sample_rate": 44100}
+
+
+def reference_audio_combination():
+    collector, _, _ = ref_collector.load()
+    node = collector.DistributedCollectorNode()
+    return [fingerprint(node._combine_audio(master, workers, EMPTY_AUDIO, order)) for master, workers, order in _audio_cases()]
+
+
+def test_audio_combination_matches_reference():
+    """nodes/collector.py:121-174 (the reference's _combine_audio) against our combine_audio on the same piece sets."""
+    from __graft_entry__ import load_package
+    load_package()
+    from comfyui_distributed_b200.nodes.collector import combine_audio
+    want = reference_fingerprints("test_collector_vs_reference")["combine_audio"]
+    cases = list(_audio_cases())
+    assert len(want) == len(cases)
+    for (master, workers, order), ref in zip(cases, want):
         seq = [master] + [workers.get(w) for w in order] + [workers[w] for w in sorted(workers) if w not in order]
-        got = combine_audio(seq, empty)
+        got = fingerprint(combine_audio(seq, EMPTY_AUDIO))
         assert got["sample_rate"] == ref["sample_rate"]
-        assert torch.equal(got["waveform"], ref["waveform"])
+        assert got["waveform"] == ref["waveform"]

@@ -2,7 +2,9 @@
 reference's own process_tiles_batch (upscale/tile_ops.py:239-287), both against the same recording
 stand-in for ComfyUI's `nodes` module: the sampler must be called with the same pixels, seed/steps/cfg/...,
 the same cropped ControlNet hints / areas / GLIGEN boxes, the same tile-local model patch, in the same
-order, and hand back the same pixels.  CPU only; needs /root/reference (skipped on the GPU box)."""
+order, and hand back the same pixels.  CPU only.  What the reference's side saw and returned is stored in
+tests/golden/reference_fingerprints.json; reference_process_tiles_batch recomputes it where the reference tree is
+loadable (oracle/gen_reference_fingerprints.py)."""
 import copy
 import sys
 import types
@@ -12,14 +14,12 @@ import torch
 
 import ref_loader
 from __graft_entry__ import load_package
+from inputs import fingerprint, reference_fingerprints
 
 load_package()
 from comfyui_distributed_b200 import planner  # noqa: E402
 from comfyui_distributed_b200.conditioning import make_cond_cropper  # noqa: E402
 from comfyui_distributed_b200.denoise import ComfySampler  # noqa: E402
-
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
-
 
 class FakeControl:
     def __init__(self, hint, prev=None):
@@ -88,18 +88,13 @@ def _recording_nodes(log, tiled=()):
     return ns
 
 
-def _same(a, b):
-    if isinstance(a, torch.Tensor):
-        return isinstance(b, torch.Tensor) and a.shape == b.shape and torch.equal(a, b)
-    if isinstance(a, (list, tuple)):
-        return isinstance(b, (list, tuple)) and len(a) == len(b) and all(_same(x, y) for x, y in zip(a, b))
-    return a == b
+CASES = [(700, 520, 256, 32, True), (420, 300, 128, 16, False)]
+TILED = [(False, ()), (True, ("encode", "decode")), (True, ("decode",)), (True, ())]
 
 
-@pytest.mark.parametrize("tiled_decode,tiled", [(False, ()), (True, ("encode", "decode")), (True, ("decode",)), (True, ())])
-@pytest.mark.parametrize("W,H,tile,pad,uniform", [(700, 520, 256, 32, True), (420, 300, 128, 16, False)])
-def test_sampler_driver_matches_process_tiles_batch(monkeypatch, W, H, tile, pad, uniform, tiled_decode, tiled):
-    tile_ops, _, _ = ref_loader.load()
+def _side(side, W, H, tile, pad, uniform, tiled_decode, tiled):
+    """Every tile of the plan through one side ("ref": the reference's process_tiles_batch, "new": ComfySampler)
+    -> [(tile index, returned pixels, calls the recording `nodes` saw)]."""
     g = torch.Generator().manual_seed(1)
     B = 2
     hint = torch.rand(1, 3, H // 2, W // 2, generator=g)
@@ -114,25 +109,52 @@ def test_sampler_driver_matches_process_tiles_batch(monkeypatch, W, H, tile, pad
 
     p = planner.Plan.build(W, H, tile, tile, pad, 8, uniform)
     args = (123, 7, 4.5, "euler", "normal", 0.35)
+    tile_ops = ref_loader.load()[0] if side == "ref" else None
+    res = []
     for t in p.tiles:
         px = torch.rand(B, t.ph, t.pw, 3, generator=g)
-        logs = {}
-        outs = {}
-        for side in ("ref", "new"):
-            logs[side] = []
-            monkeypatch.setitem(sys.modules, "nodes", _recording_nodes(logs[side], tiled))
+        log = []
+        saved = sys.modules.get("nodes")
+        sys.modules["nodes"] = _recording_nodes(log, tiled)
+        try:
             model = Model(DiffSynthCnetPatch("mp", None, control_image.clone(), 1.0))
             pos, neg = make_cond(), make_cond()
             if side == "ref":
-                node = tile_ops.TileOpsMixin()
-                outs[side] = node.process_tiles_batch(px.clone(), model, pos, neg, "vae", *args, tiled_decode,
-                                                      (t.x1, t.y1, t.x2, t.y2), (W, H))
+                out = tile_ops.TileOpsMixin().process_tiles_batch(px.clone(), model, pos, neg, "vae", *args, tiled_decode,
+                                                                  (t.x1, t.y1, t.x2, t.y2), (W, H))
             else:
                 s = ComfySampler(model, pos, neg, "vae", *args, tiled_decode=tiled_decode, image_size=(W, H),
                                  cond_cropper=make_cond_cropper())
-                outs[side] = s(px.clone()[None], [t])[0]
-            assert torch.equal(model.patch.image, control_image)          # patch restored on both sides
-        assert torch.equal(outs["ref"], outs["new"])
-        assert len(logs["ref"]) == len(logs["new"]) == 3
-        for a, b in zip(logs["ref"], logs["new"]):
-            assert a[0] == b[0] and _same(a[1:], b[1:]), (t.idx, a[0])
+                out = s(px.clone()[None], [t])[0]
+        finally:
+            if saved is None:
+                sys.modules.pop("nodes", None)
+            else:
+                sys.modules["nodes"] = saved
+        assert torch.equal(model.patch.image, control_image)          # patch restored after the tile
+        res.append((t.idx, out, log))
+    return res
+
+
+def _key(W, H, tile, pad, uniform, tiled_decode, tiled):
+    return repr((W, H, tile, pad, uniform, tiled_decode, tiled))
+
+
+def reference_process_tiles_batch(W, H, tile, pad, uniform, tiled_decode, tiled):
+    return [{"idx": i, "out": fingerprint(out), "log": [fingerprint(c) for c in log]}
+            for i, out, log in _side("ref", W, H, tile, pad, uniform, tiled_decode, tiled)]
+
+
+@pytest.mark.parametrize("tiled_decode,tiled", TILED)
+@pytest.mark.parametrize("W,H,tile,pad,uniform", CASES)
+def test_sampler_driver_matches_process_tiles_batch(W, H, tile, pad, uniform, tiled_decode, tiled):
+    want = reference_fingerprints("test_comfy_sampler_vs_reference")["process_tiles_batch"][
+        _key(W, H, tile, pad, uniform, tiled_decode, tiled)]
+    got = _side("new", W, H, tile, pad, uniform, tiled_decode, tiled)
+    assert len(got) == len(want)
+    for (idx, out, log), w in zip(got, want):
+        assert idx == w["idx"]
+        assert fingerprint(out) == w["out"], idx
+        assert len(log) == len(w["log"]) == 3
+        for call, wc in zip(log, w["log"]):
+            assert fingerprint(call) == wc, (idx, call[0])

@@ -182,7 +182,8 @@ def _w_shared_host(rank, world):
     import glob
     sh = udist.SharedHost.get(None)
     sh.MAX_MAPPED = 3
-    assert not sh.pin                                     # no device here: the hand-shakes and the mapping policy only
+    assert sh.pin == torch.cuda.is_available()            # buffers are page-locked wherever there is a device
+    sh.pin = False                                        # the hand-shakes and the mapping policy only, with or without one
     held = None
     rows = [100, 200, 100, 300, 400, 500, 100, 200]
     for j, n in enumerate(rows):

@@ -1,6 +1,6 @@
-"""Tile-local model patches == the reference's crop_model_cond (utils/crop_model_patch.py), run side
-by side on the same fake ComfyUI objects (needs /root/reference; skipped on the GPU box), plus
-behaviour checks that run everywhere."""
+"""Tile-local model patches == the reference's crop_model_cond (utils/crop_model_patch.py) on the same fake
+ComfyUI objects (what the reference computed: tests/golden/reference_fingerprints.json, recomputed by
+reference_crop_model_cond where the reference tree is loadable), plus behaviour checks."""
 import sys
 
 import pytest
@@ -8,6 +8,7 @@ import torch
 
 import ref_loader
 from __graft_entry__ import load_package
+from inputs import fingerprint, reference_fingerprints
 
 load_package()
 from comfyui_distributed_b200 import model_patch as MP  # noqa: E402
@@ -92,21 +93,28 @@ def test_patch_shared_by_two_blocks_is_cropped_once():
         assert DiffSynthCnetPatch.inits == n0 + 1        # re-initialised once although registered twice
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
+def _seen(ctx):
+    torch.manual_seed(0)
+    model, p, img = _setup()
+    with ctx(model):
+        seen = (p.image.clone(), p.encoded_image.clone(), tuple(p.encoded_image_size))
+    return seen, p, img
+
+
+def reference_crop_model_cond(latent_crop, region, canvas):
+    ref_loader.load()
+    R = sys.modules[ref_loader.PKG + ".utils.crop_model_patch"]
+    seen, _, _ = _seen(lambda m: R.crop_model_cond(m, region, canvas, canvas, (544, 544), latent_crop=latent_crop))
+    return fingerprint(seen)
+
+
 @pytest.mark.parametrize("latent_crop", [False, True])
 @pytest.mark.parametrize("region,canvas", [(REGION, CANVAS), ((0, 0, 544, 544), (1300, 1100)), ((724, 524, 1300, 1100), (1300, 1100))])
 def test_matches_reference_crop_model_cond(latent_crop, region, canvas):
-    ref_loader.load()
-    R = sys.modules[ref_loader.PKG + ".utils.crop_model_patch"]
-    seen = {}
-    for name, ctx in (("ref", lambda m: R.crop_model_cond(m, region, canvas, canvas, (544, 544), latent_crop=latent_crop)),
-                      ("new", lambda m: MP.cropped_model_patches(m, region, canvas, latent_crop=latent_crop))):
-        torch.manual_seed(0)
-        model, p, img = _setup()
-        with ctx(model):
-            seen[name] = (p.image.clone(), p.encoded_image.clone(), tuple(p.encoded_image_size))
-        if name == "new":
-            assert torch.equal(p.image, img)
-    assert torch.equal(seen["ref"][0], seen["new"][0])
-    assert torch.equal(seen["ref"][1], seen["new"][1])
-    assert seen["ref"][2] == seen["new"][2]
+    seen, p, img = _seen(lambda m: MP.cropped_model_patches(m, region, canvas, latent_crop=latent_crop))
+    assert torch.equal(p.image, img)
+    want = reference_fingerprints("test_model_patch")["crop_model_cond"][repr((latent_crop, region, canvas))]
+    got = fingerprint(seen)
+    assert got["tuple"][0] == want["tuple"][0]
+    assert got["tuple"][1] == want["tuple"][1]
+    assert got["tuple"][2] == want["tuple"][2]
